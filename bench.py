@@ -4,6 +4,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
                     [--gar trmean --nb-workers 25 --nb-byz 10 --dim 1310922] [--no-sweep]
+                    [--dump-outputs DIR]
 
 A "step" is ONE aggregation call over one stack of n worker gradients (fp32, length d per
 GPU).  Default workload = BASELINE.json configs[1]: trimmed mean, n=25, f=10, d=1,310,922
@@ -20,9 +21,15 @@ One JSON line is printed by rank 0 (see the driver contract in the task statemen
   e2e         the same metric through the reference-facing call `gars[gar](gradients=<host
               tensors>, f=f)`: pinned host rows -> H2D -> kernel -> D2H of the result, per step
   cpu_baseline  the UNMODIFIED reference's `aggregators.gars[gar].unchecked` on CPU tensors, on the host
-                cores (baseline/_ref; the port oracle/refcost.py only when no reference is present)
+                cores (the checkout named by $BYZ_REFERENCE; without one, its port oracle/refcost.py)
   sweep       (N=1) kernel time / GB/s / roofline fraction of the other rules and sizes
 `--impl reference` times the reference's CPU aggregation alone, on the same workload.
+`--steps K` is the number of timed steps of every timed loop: the headline region, the plugin and e2e
+calls and the sharded block (the sweep keeps the median of 7-15 samples per point).
+`--dump-outputs DIR` writes what the last timed step returned as DIR/aggregate.npy (fp32; with N > 1
+each rank writes DIR/aggregate_rank<r>.npy).  The inputs are seeded, so two builds run with the same
+arguments can be compared output for output.  Above 60 MB in all, a fixed seeded sample of the
+elements is written instead, with their positions in DIR/<name>_index.npy (fp64).
 """
 
 import argparse
@@ -36,6 +43,9 @@ import time
 
 ROOT = pathlib.Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True     # the tree may be read-only: leave nothing in it
+
+DUMP_BYTES = 60_000_000         # --dump-outputs: under 64 MB with the .npy headers
 
 L2_BYTES = 126 * 1024 * 1024
 FALLBACK_HBM_GBS = 6650.0   # /opt/skills/guides/B200_PROFILING.md, used only without MEASURED_PEAKS.json
@@ -129,23 +139,39 @@ def call_device(bz, sharded, gar, rows, f, world):
 
 def time_steps(torch, fn, steps, pairs=True):
   """ K steps on the current stream between two CUDA events; with `pairs`, also one event pair
-  around every step (per-launch durations).  Returns (total_ms, per_step_ms list or None). """
+  around every step (per-launch durations).  Returns (total_ms, per_step_ms list or None, what
+  the last step returned). """
   if not pairs:
     a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     a.record()
     for k in range(steps):
-      fn(k)
+      out = fn(k)
     b.record()
     torch.cuda.synchronize()
-    return a.elapsed_time(b), None
+    return a.elapsed_time(b), None, out
   ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
   for k in range(steps):
     ev[k][0].record()
-    fn(k)
+    out = fn(k)
     ev[k][1].record()
   torch.cuda.synchronize()
   total = ev[0][0].elapsed_time(ev[-1][1])
-  return total, [a.elapsed_time(b) for a, b in ev]
+  return total, [a.elapsed_time(b) for a, b in ev], out
+
+def dump_outputs(directory, outputs):
+  """ Each array of `outputs` (name -> NumPy array) as <directory>/<name>.npy, DUMP_BYTES in all at most:
+  an array over its share is replaced by a sample of its elements at fixed seeded positions, which go
+  to <name>_index.npy. """
+  import numpy as np
+  os.makedirs(directory, exist_ok=True)
+  share = DUMP_BYTES // max(len(outputs), 1)
+  for name, value in outputs.items():
+    value = np.ascontiguousarray(value).reshape(-1)
+    if value.nbytes > share:
+      index = np.sort(np.random.default_rng(0).choice(value.size, share // (value.itemsize + 8), replace=False))
+      np.save(os.path.join(directory, name + "_index.npy"), index.astype(np.float64))
+      value = value[index]
+    np.save(os.path.join(directory, name + ".npy"), value)
 
 def peak_hbm():
   path = ROOT / "MEASURED_PEAKS.json"
@@ -179,8 +205,8 @@ def cpu_info():
 
 def reference_callable(gar):
   """ (fn(rows, f), kind, path): the UNMODIFIED reference's `aggregators.gars[gar].unchecked`
-  (BASELINE.md §4.2; search order $BYZ_REFERENCE, baseline/_ref, /root/reference) — nothing of this
-  repository is on that path — or, only when no reference checkout is present, the port of its
+  (BASELINE.md §4.2; the checkout named by $BYZ_REFERENCE) — nothing of this repository is on
+  that path — or, only when no reference checkout is given, the port of its
   ATen operator sequence (oracle/refcost.py). """
   from oracle import reference
   root, aggregators = reference.load()
@@ -271,7 +297,7 @@ def timed_max_over_ranks(torch, dist, device, fn, steps, warmup=5):
     ms = float(t.item())
   return ms / steps * 1e3
 
-def sharded_block(torch, dist, bz, sharded, device, world, rank, peak):
+def sharded_block(torch, dist, bz, sharded, device, world, rank, peak, steps):
   """ The multi-GPU path BASELINE.json's north_star names (SURVEY §8(e)), timed on the device:
     collective  Multi-Krum + Bulyan at C3 (n = 25, f = 5, d = 1,310,922 PER GPU: weak scaling)
                 through the prepared sharded call: with the NCCL all-gather of the R n x n blocks
@@ -282,7 +308,6 @@ def sharded_block(torch, dist, bz, sharded, device, world, rank, peak):
     c4_strong   median + trimmed mean at C4 (n = 51, f = 12, d = 36,546,980 TOTAL, split over the
                 N ranks: strong scaling; no collective on this path). """
   out = dict(world=world)
-  steps = 200
   # ---- collective path, weak scaling --------------------------------------------------------------
   n, f, d = 25, 5, 1_310_922
   sets = 4                                           # 4 x 131 MB > 3 x L2
@@ -312,7 +337,7 @@ def sharded_block(torch, dist, bz, sharded, device, world, rank, peak):
   try:
     params = torch.zeros(world * d, device=device)
     shard = torch.randn(d, device=device, generator=gen)
-    upd_us = timed_max_over_ranks(torch, dist, device, lambda k: sharded.apply_update(params, shard, 0.01, weight_decay=1e-4), 50)
+    upd_us = timed_max_over_ranks(torch, dist, device, lambda k: sharded.apply_update(params, shard, 0.01, weight_decay=1e-4), steps)
     out["model_update"] = dict(what="sharded.apply_update: p -= lr (g + w p) on this rank's d columns, then ONE all-gather of the parameters (experiments/model.py:368-380 for a d-sharded trainer)",
                                d_total=world * d, us_per_step=upd_us, allgather_bytes_per_rank=d * 4)
     del params, shard
@@ -332,7 +357,7 @@ def sharded_block(torch, dist, bz, sharded, device, world, rank, peak):
   rows = []
   for gar in ("median", "trmean"):
     plans = [sharded.ShardedPlan(gar, st, f=f) for st in stacks]
-    us = timed_max_over_ranks(torch, dist, device, lambda k: plans[k % sets](), 20 if world == 1 else 50, warmup=3)
+    us = timed_max_over_ranks(torch, dist, device, lambda k: plans[k % sets](), steps, warmup=3)
     alg = (n + 1) * total * 4
     rows.append(dict(gar=gar, n=n, f=f, d_total=total, d_this_rank=d, us_per_step=us, params_per_s=total / (us * 1e-6),
                      aggregate_gbs=alg / (us * 1e-6) / 1e9, hbm_frac_per_gpu=alg / world / (us * 1e-6) / 1e9 / peak))
@@ -411,9 +436,11 @@ def run_b200(args):
     step(k)
   barrier()
   with ClockSampler(local) as clocks:
-    total_ms, _ = time_steps(torch, step, args.steps, pairs=False)     # THE timed region: K steps, two events
+    total_ms, _, last = time_steps(torch, step, args.steps, pairs=False)     # THE timed region: K steps, two events
+    if args.dump_outputs:
+      dumped = last.detach().cpu().numpy()
     barrier()
-    _, per_step = time_steps(torch, step, args.steps, pairs=True)      # second pass: per-launch durations
+    _, per_step, _ = time_steps(torch, step, args.steps, pairs=True)      # second pass: per-launch durations
     barrier()
     # keep the sampler alive a little when the region is very short
     # (a FIXED number of extra steps: every rank must issue the same collectives)
@@ -452,13 +479,13 @@ def run_b200(args):
     for k in range(3):
       plugin_step(k)
     barrier()
-    plugin_total, _ = time_steps(torch, plugin_step, min(args.steps, 100))
-    plugin_ms = plugin_total / min(args.steps, 100)
+    plugin_total, _, _ = time_steps(torch, plugin_step, args.steps)
+    plugin_ms = plugin_total / args.steps
   else:
     plugin_ms = None
 
   # ---- end to end through the reference-facing call with HOST buffers ---------------------------
-  e2e_steps = max(3, min(args.steps, 20))
+  e2e_steps = args.steps
   host_sets = 2
   # pinned host buffers, allocated while bound to the GPU-local CPUs (first touch puts the pages on
   # the GPU's NUMA node: a copy from the other socket runs at a fraction of the PCIe rate)
@@ -471,7 +498,7 @@ def run_b200(args):
   for k in range(12):             # the engine measures its host->device candidates during the first calls (engine._HostPath)
     e2e_step(k)
   barrier()
-  e2e_total, e2e_each = time_steps(torch, e2e_step, e2e_steps)
+  e2e_total, e2e_each, _ = time_steps(torch, e2e_step, e2e_steps)
   if dist is not None:
     t = torch.tensor([e2e_total], device=device, dtype=torch.float64)
     dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -514,9 +541,11 @@ def run_b200(args):
       line["sweep"] = sweep(torch, bz, device, peak)
   if not args.no_sharded:
     try:
-      line["sharded"] = sharded_block(torch, dist, bz, sharded, device, world, rank, peak)
+      line["sharded"] = sharded_block(torch, dist, bz, sharded, device, world, rank, peak, args.steps)
     except Exception as err:
       line["sharded"] = dict(error=f"{type(err).__name__}: {err}"[:300])
+  if args.dump_outputs:
+    dump_outputs(args.dump_outputs, {"aggregate" if world == 1 else f"aggregate_rank{rank}": dumped})
   if rank == 0:
     print(json.dumps(line), flush=True)
   if dist is not None:
@@ -610,7 +639,13 @@ def main():
   ap.add_argument("--no-sharded", action="store_true", help="skip the `sharded` block (collective path at C3 per GPU + C4 strong scaling; at N = 1 it is the reference line of the series)")
   ap.add_argument("--exchange", choices=("auto", "nccl", "p2p"), default="auto",
                   help="N > 1, distance-based rules: all-gather (NCCL) or blocks read in place over NVLink peer memory")
+  ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                  help="write what the last timed step returned to DIR/<name>.npy (b200 implementation)")
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error("--steps must be at least 1")
+  if args.dump_outputs and args.impl != "b200":
+    ap.error("--dump-outputs writes the outputs of the b200 implementation")
   global EXCHANGE
   EXCHANGE = args.exchange
   if args.impl == "reference":

@@ -4,10 +4,8 @@
 Only `tests/`, `__graft_entry__.smoke()` and `bench.py`'s CPU legs (`--impl reference`,
 `cpu_baseline`) may import this module; nothing under `byzantinemomentum_b200/` does.
 
-Search order (BASELINE.md §4.2): `$BYZ_REFERENCE`, `<repo>/baseline/_ref` (a verbatim copy made by
-`tools/install_ref.sh`; git-ignored, but it travels to the GPU box with the gpurun snapshot),
-`/root/reference` (build container only).  A candidate counts when it holds
-`aggregators/__init__.py` and `attack.py`.
+The reference is found through `$BYZ_REFERENCE`, the root of a ByzantineMomentum checkout; it is
+never part of this repository.  A root counts when it holds `aggregators/__init__.py` and `attack.py`.
 
 Importing the reference's `tools` package rewires `sys.stdout`, `sys.stderr` and `sys.excepthook`
 (tools/__init__.py:215-216,246); `load()` restores them, so a test or the bench keeps its own
@@ -24,12 +22,7 @@ ROOT = pathlib.Path(__file__).resolve().parent.parent
 
 def candidates():
   env = os.environ.get("BYZ_REFERENCE")
-  out = []
-  if env:
-    out.append(pathlib.Path(env))
-  out.append(ROOT / "baseline" / "_ref")
-  out.append(pathlib.Path("/root/reference"))
-  return out
+  return [pathlib.Path(env)] if env else []
 
 def find_root():
   """ Root of the first usable reference checkout, or None. """

@@ -15,11 +15,11 @@ if str(ROOT) not in sys.path:
 GOLDEN_DIR = ROOT / "tests" / "golden"
 
 def reference_root():
-  """ Root of the unmodified reference ($BYZ_REFERENCE, baseline/_ref, /root/reference) or None. """
+  """ Root of the unmodified reference checkout named by $BYZ_REFERENCE, or None. """
   from oracle import reference
   return reference.find_root()
 
-needs_reference = pytest.mark.skipif(reference_root() is None, reason="no reference checkout on this box (tools/install_ref.sh)")
+needs_reference = pytest.mark.skipif(reference_root() is None, reason="needs a reference checkout: set BYZ_REFERENCE")
 
 def pytest_configure(config):
   config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with `-m gpu`)")

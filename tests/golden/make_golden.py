@@ -179,12 +179,27 @@ def run_case(name, kind, n, nb, d, seed, fs):
   out["manifest"] = np.array(json.dumps(manifest))
   return out
 
+# Other seeds and shapes than CASES, kept apart under live/ (tests/test_oracle_live_reference.py):
+# (name, kind, n, nb_byz, d, seed, fs), three seeds each
+LIVE_CASES = [
+  ("live_iid_n13", "iid", 13, 3, 211, 9001, [1, 2, 3, 5]),
+  ("live_empire_n17", "empire", 17, 4, 333, 9002, [2, 3, 4, 7]),
+  ("live_little_n10", "little", 10, 2, 97, 9003, [1, 2, 3]),
+  ("live_nan_n9", "nan", 9, 2, 65, 9004, [1, 2, 3]),
+  ("live_inf_n15", "inf", 15, 3, 130, 9005, [1, 3, 5]),
+  ("live_quant_n21", "quant", 21, 4, 96, 9006, [2, 4, 9]),
+  ("live_iid_n40", "iid", 40, 9, 75, 9007, [3, 9, 18]),
+]
+LIVE_CASES = [(f"{name}_s{k}", kind, n, nb, d + 7 * k, seed + 100 * k, fs) for (name, kind, n, nb, d, seed, fs) in LIVE_CASES for k in range(3)]
+
 def main():
+  """ `make_golden.py` writes CASES, `make_golden.py --live` writes LIVE_CASES under live/. """
   torch.set_num_threads(1)  # thread-count independent results where ATen's order depends on it
+  live = sys.argv[1:] == ["--live"]
   total = 0
-  for case in CASES:
+  for case in (LIVE_CASES if live else CASES):
     data = run_case(*case)
-    path = HERE / f"golden_{case[0]}.npz"
+    path = (HERE / "live" if live else HERE) / f"golden_{case[0]}.npz"
     np.savez_compressed(path, **data)
     total += path.stat().st_size
     man = json.loads(str(data["manifest"]))

@@ -1,8 +1,8 @@
 # coding: utf-8
 """The drop-in INSIDE the unmodified reference, on the GPU (VERDICT r1 weak #1, SURVEY §8 a16/b).
 
-`tools/drive_attack.py` executes the reference's own `attack.py` (from `baseline/_ref`, copied
-verbatim by `tools/install_ref.sh`; nothing of it is edited) with `runpy`, synthetic batches in
+`tools/drive_attack.py` executes the reference's own `attack.py` (from the checkout named by
+$BYZ_REFERENCE: skipped without one; nothing of it is edited) with `runpy`, synthetic batches in
 place of the dataset download, and the CUDA rules registered through the reference's own
 `aggregators.register` (`b200-<name>`) and through the `native.<rule>.aggregate` hook it probes
 (`native-<name>`).  Everything of attack.py:799-827 then runs against the CUDA rules on cuda:0:

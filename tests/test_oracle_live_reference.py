@@ -1,55 +1,20 @@
 # coding: utf-8
-"""Beyond the committed goldens: generate FRESH reference outputs (other seeds, other shapes) with
-the golden generator and check the oracle against them with the same comparisons.  Build
-container only (needs /root/reference); the generator runs in a subprocess because importing the
-reference rewires sys.stdout / sys.stderr (tools/__init__.py:215-216,246)."""
+"""Beyond the committed goldens: reference outputs for other seeds and shapes (`tests/golden/live/`,
+written by `tests/golden/make_golden.py --live` from the unmodified reference), checked against the
+oracle with the same comparisons as the goldens."""
 
-import os
 import pathlib
-import subprocess
-import sys
-
-import pytest
 
 import conftest
 from test_oracle_golden import test_oracle_matches_reference as check_call
 
-ROOT = pathlib.Path(__file__).resolve().parent.parent
-REF = conftest.reference_root() or pathlib.Path("/nonexistent")
+LIVE_DIR = pathlib.Path(__file__).resolve().parent / "golden" / "live"
 
-# (name, kind, n, nb_byz, d, seed, fs) — none of them is a committed fixture
-LIVE_CASES = [
-  ("live_iid_n13", "iid", 13, 3, 211, 9001, [1, 2, 3, 5]),
-  ("live_empire_n17", "empire", 17, 4, 333, 9002, [2, 3, 4, 7]),
-  ("live_little_n10", "little", 10, 2, 97, 9003, [1, 2, 3]),
-  ("live_nan_n9", "nan", 9, 2, 65, 9004, [1, 2, 3]),
-  ("live_inf_n15", "inf", 15, 3, 130, 9005, [1, 3, 5]),
-  ("live_quant_n21", "quant", 21, 4, 96, 9006, [2, 4, 9]),
-  ("live_iid_n40", "iid", 40, 9, 75, 9007, [3, 9, 18]),
-]
-
-LIVE_CASES = [(f"{name}_s{k}", kind, n, nb, d + 7 * k, seed + 100 * k, fs) for (name, kind, n, nb, d, seed, fs) in LIVE_CASES for k in range(3)]
-
-SCRIPT = r"""
-import sys, json, numpy as np
-sys.path.insert(0, {golden_dir!r})
-import make_golden
-import torch
-torch.set_num_threads(1)
-for case in {cases!r}:
-  data = make_golden.run_case(*case)
-  np.savez_compressed({out_dir!r} + "/golden_" + case[0] + ".npz", **data)
-"""
-
-@pytest.mark.skipif(not (REF / "aggregators" / "__init__.py").exists(), reason="reference not present on this box")
-def test_oracle_matches_fresh_reference_outputs(tmp_path):
-  script = tmp_path / "gen.py"
-  script.write_text(SCRIPT.format(golden_dir=str(ROOT / "tests" / "golden"), cases=LIVE_CASES, out_dir=str(tmp_path)))
-  proc = subprocess.run([sys.executable, str(script)], cwd=tmp_path, capture_output=True, text=True, timeout=900,
-                        env=dict(os.environ, BYZ_REFERENCE=str(REF)))
-  assert proc.returncode == 0, proc.stdout[-2000:] + proc.stderr[-3000:]
+def test_oracle_matches_fresh_reference_outputs():
+  paths = sorted(LIVE_DIR.glob("golden_live_*.npz"))
+  assert len(paths) == 21, [p.name for p in paths]
   checked = 0
-  for path in sorted(tmp_path.glob("golden_live_*.npz")):
+  for path in paths:
     golden = conftest.Golden(path)
     for call in golden.calls:
       check_call(golden, call)

@@ -1,8 +1,13 @@
 # coding: utf-8
-"""Drop-in registration inside the UNMODIFIED reference (build container only: skipped where
-/root/reference does not exist, e.g. on the GPU box).  Runs in a subprocess because importing
-the reference replaces sys.stdout / sys.stderr / sys.excepthook (tools/__init__.py:215-216,246)."""
+"""Drop-in registration inside the UNMODIFIED reference.  The tests run against the checkout named by
+$BYZ_REFERENCE and, without one, against `tests/standin/`: a stand-in written for these tests with
+the reference's registry, `tools`, `experiments` and attack.py interfaces, whose stock rules answer
+`check()` and `upper_bound()` as the reference did.  What the reference's `check()`, `upper_bound()`
+and attack.py hold is recorded in `tests/golden/reference_checks.json`
+(tests/golden/make_check_golden.py).  They run in a subprocess because importing the reference
+replaces sys.stdout / sys.stderr / sys.excepthook (tools/__init__.py:215-216,246)."""
 
+import json
 import os
 import pathlib
 import subprocess
@@ -13,7 +18,33 @@ import pytest
 import conftest
 
 ROOT = pathlib.Path(__file__).resolve().parent.parent
-REF = conftest.reference_root() or pathlib.Path("/nonexistent")
+STANDIN = ROOT / "tests" / "standin"
+REF = conftest.reference_root() or STANDIN
+
+def check_grid():
+  """ (rule, n, f, extra keyword arguments) on which the rules' `check()` verdicts are compared. """
+  return [(name, n, f, extra) for n in (1, 3, 7, 11, 25) for f in (0, 1, 2, 3, 5, 12, "x")
+          for name in ("trmean", "phocas", "meamed", "krum", "bulyan", "brute", "aksel", "cge", "median", "average")
+          for extra in ({}, {"m": 1}, {"m": 99}, {"mode": "n-f"}, {"mode": "zzz"})]
+
+def test_checks_and_upper_bound_match_the_reference():
+  """ The CUDA rules accept exactly the (n, f, extra) the reference's own check() accepts, and
+  Multi-Krum's upper bound is the reference's (study.py:361-366 reads it). """
+  import torch
+  import byzantinemomentum_b200 as bz
+  recorded = json.loads((conftest.GOLDEN_DIR / "reference_checks.json").read_text())
+  want = {json.dumps(entry) for entry in recorded["accepted"]}
+  assert len(want) > 100, len(want)
+  differs = []
+  for name, n, f, extra in check_grid():
+    try:
+      got = bz.gars[name].check(gradients=[torch.zeros(4) for _ in range(n)], f=f, **extra) is None
+    except TypeError:
+      got = False
+    if got != (json.dumps([name, n, f, extra]) in want):
+      differs.append((name, n, f, extra, got))
+  assert not differs, differs[:10]
+  assert bz.gars["krum"].upper_bound(25, 5, 10) == recorded["krum_upper_bound_25_5_10"]
 
 SCRIPT = r"""
 import sys
@@ -73,7 +104,6 @@ out.write("RESULT " + " ".join(str(int(x)) for x in res) + "\n")
 out.flush()
 """
 
-@pytest.mark.skipif(not (REF / "aggregators" / "__init__.py").exists(), reason="reference not present on this box")
 def test_rules_register_inside_the_unmodified_reference(tmp_path):
   script = tmp_path / "drive.py"
   script.write_text(SCRIPT.format(root=str(ROOT), ref=str(REF)))
@@ -91,7 +121,6 @@ def _drive(tmp_path, gar):
          "--", "--gar", gar] + ATTACK_ARGS
   return subprocess.run(cmd, cwd=tmp_path, capture_output=True, text=True, timeout=600)
 
-@pytest.mark.skipif(not (REF / "attack.py").exists(), reason="reference not present on this box")
 def test_unmodified_attack_py_runs_offline_with_the_rules_registered(tmp_path):
   """ SURVEY.md §8(b): the runpy recipe.  The stock rule drives two full steps (synthetic data,
   study metrics through the swapped `compute_avg_dev_max`), with every b200-<name> registered. """
@@ -100,7 +129,6 @@ def test_unmodified_attack_py_runs_offline_with_the_rules_registered(tmp_path):
   assert "registered: b200-average" in proc.stdout and "b200-cge" in proc.stdout
   assert "Training..." in proc.stdout
 
-@pytest.mark.skipif(not (REF / "attack.py").exists(), reason="reference not present on this box")
 def test_cuda_rule_inside_attack_py_fails_loudly_without_a_gpu(tmp_path):
   """ No CPU fallback: selecting a CUDA rule on a box without a GPU stops attack.py with the
   library's error instead of silently computing on the host. """
@@ -111,16 +139,23 @@ def test_cuda_rule_inside_attack_py_fails_loudly_without_a_gpu(tmp_path):
   assert proc.returncode != 0
   assert "no CUDA device available" in proc.stdout + proc.stderr
 
-@pytest.mark.skipif(not (REF / "attack.py").exists(), reason="reference not present on this box")
-def test_in_memory_rewrites_of_attack_py_match_their_anchors_and_compile():
+def test_in_memory_rewrites_of_attack_py_match_their_anchors_and_compile(monkeypatch):
   """ tools/drive_attack.py --fuse-gradients / --fuse-study: every anchor is found exactly as often as
   expected in the reference's attack.py, the study block has the known digest, the rewritten source
   compiles and calls the helper; a source that differs is refused. """
+  import hashlib
   import importlib.util
   spec = importlib.util.spec_from_file_location("drive_attack", ROOT / "tools" / "drive_attack.py")
   drive = importlib.util.module_from_spec(spec)
   spec.loader.exec_module(drive)
+  sha = lambda text: hashlib.sha256(text.encode()).hexdigest()
+  recorded = json.loads((conftest.GOLDEN_DIR / "reference_checks.json").read_text())["attack_py"]
+  expected = {drive.CLIP_AND_CLONE: 2, drive.MOMENTUM: 1, drive.STUDY_BEGIN: 1, drive.STUDY_END: 1}
+  assert {sha(text): count for text, count in expected.items()} == {k: v for k, v in recorded.items() if k != "study_block"}
+  assert drive.STUDY_SHA256 == recorded["study_block"]
   source = (REF / "attack.py").read_text()
+  if REF == STANDIN:          # the stand-in's study block is its own text, not the reference's
+    monkeypatch.setattr(drive, "STUDY_SHA256", sha(source[source.index(drive.STUDY_BEGIN):source.index(drive.STUDY_END)]))
   both = drive.rewrite(source, True, True)
   compile(both, "attack.py", "exec")
   assert both.count("__bz_rows.push(") == 2 and both.count("__bz_rows.study(") == 1
